@@ -123,6 +123,25 @@ def kernel_family(name):
     return name.split(" ")[0]
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays, seed=0):
+    """Write each array as <dirname>/<name>.npy in float32.  An array larger than its share of DUMP_BYTES is cut to a fixed,
+    seeded sample of its leading-axis rows (whole utterances), kept in order, so two builds dump the same rows."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() * 4 > budget:
+            k = budget // (a[0].numel() * 4)
+            assert k >= 1, f"one row of {name} is larger than the {budget} B dump budget"
+            rows = torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(seed))[:k].sort().values
+            a = a[rows]
+        np.save(os.path.join(dirname, name + ".npy"), a.numpy())
+
+
 def run_ours(args):
     from styletts2_b200 import lib
     from styletts2_b200 import ops as _ops
@@ -206,9 +225,12 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(devin)
+        wav_last = step(devin)
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        # the waveform of the last timed step, read before anything else runs (under --graph it is the graph's output buffer)
+        dump_outputs(args.dump_outputs, {"wav": wav_last.view(B, L)})
     launches = lib.launch_count() - n0
     if args.graph:
         launches = graph_launches[0] * args.steps   # kernels of this library inside the replayed CUDA graph x replays
@@ -474,7 +496,14 @@ def main():
     ap.add_argument("--no-graph", dest="graph", action="store_false", help="eager launches instead of one CUDA graph per step")
     ap.add_argument("--dump-launches", default=None, help="write the per-shape launch table (CUDA events, eager passes) to this JSON file")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only (ncu): device-resident loop, no JSON contract line")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the waveform [B, samples] of the last timed step to DIR/wav.npy (float32; rank 0; a fixed seeded "
+                         f"sample of whole utterances above {DUMP_BYTES >> 20} MB); same arguments -> same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

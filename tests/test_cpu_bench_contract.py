@@ -31,6 +31,24 @@ def test_reference_arm_prints_contract_line():
     assert "workload" in d["config"]
 
 
+def test_dump_outputs_writes_float32_and_samples_whole_rows_over_budget(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    wav = torch.arange(6 * 10, dtype=torch.float32).view(6, 10)
+    bench.dump_outputs(str(tmp_path / "all"), {"wav": wav})
+    a = np.load(tmp_path / "all" / "wav.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, wav.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * 10 * 4)          # room for three of the six rows
+    bench.dump_outputs(str(tmp_path / "s1"), {"wav": wav})
+    bench.dump_outputs(str(tmp_path / "s2"), {"wav": wav})
+    s1, s2 = np.load(tmp_path / "s1" / "wav.npy"), np.load(tmp_path / "s2" / "wav.npy")
+    assert s1.shape == (3, 10) and np.array_equal(s1, s2)            # fixed sample
+    rows = s1[:, 0] / 10
+    assert list(rows) == sorted(set(rows)) and all(np.array_equal(s1[i], wav.numpy()[int(r)]) for i, r in enumerate(rows))
+
+
 def test_reference_arm_nonzero_rank_exits_quietly():
     lines = _run(["--impl", "reference", "--workload", "tiny", "--steps", "1", "--warmup", "0", "--gpus", "2"],
                  env={"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2", "MASTER_ADDR": "127.0.0.1", "MASTER_PORT": "29533"})
